@@ -13,7 +13,7 @@ view-tuples x 4 views = 128 images of 256x256 (SURVEY.md section 8(d) config C4)
 through the reference-shaped public API (lib.core.function.train_integral) with
 pinned HOST batches, H2D copies and a loss read-back inside the timed region.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 --impl reference times the reference's CPU implementation of the same step
 (oracle port: torch-CPU fp32 network + numpy/OpenCV-equivalent geometry) on the
@@ -134,6 +134,27 @@ class ClockSampler(threading.Thread):
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_SAMPLE = 4_000_000      # float32 values of the model state kept by --dump-outputs (16 MB)
+
+
+def dump_outputs(out_dir, loss, model):
+    """What the last timed step handed its caller, as float32 .npy files in out_dir:
+    loss.npy (the returned loss), final_layer.{weight,bias}.npy (the updated head in full)
+    and state_sample.npy: a fixed sample (seed 0, sorted indices) of every floating-point
+    state_dict entry -- parameters after the Adam update and BatchNorm running statistics --
+    flattened and concatenated in state_dict order."""
+    os.makedirs(out_dir, exist_ok=True)
+    sd = model.state_dict()
+    out = {"loss": loss.detach().float().reshape(1),
+           "final_layer.weight": sd["final_layer.weight"], "final_layer.bias": sd["final_layer.bias"]}
+    flat = torch.cat([v.detach().reshape(-1).float() for v in sd.values() if v.is_floating_point()])
+    n = min(DUMP_SAMPLE, flat.numel())
+    idx = np.sort(np.random.default_rng(0).choice(flat.numel(), n, replace=False))
+    out["state_sample"] = flat[torch.from_numpy(idx).to(flat.device)]
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.detach().float().cpu().numpy())
+
+
 # ---------------------------------------------------------------------------- GPU arm
 def run_gpu(args):
     import torch.distributed as dist
@@ -231,6 +252,8 @@ def run_gpu(args):
         ms = tmax.item()
     ms_step = ms / args.steps
     value = world * args.tuples / (ms_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, model)    # before the eager steps below move the weights
 
     # ---- dominant kernel family (conv GEMMs): CUDA events around every launch of the same
     # step, issued eagerly right after the timed region (events cannot be read back from
@@ -537,7 +560,11 @@ def main():
                          "c5 (extra line, not the headline): R101 384x384 J17 D96, 16 tuples/GPU")
     ap.add_argument("--strong", action="store_true",
                     help="strong scaling: the tuples of ONE GPU's batch are divided among the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss and model state of the last one to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.workload == "c5":
         HW, J, D, WORKLOAD_TAG = 384, 17, 96, "C5"
         args.layers = 101

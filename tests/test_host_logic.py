@@ -722,7 +722,7 @@ def test_fused_optimizers_interchange_with_torch_optim_and_survive_rematerialisa
         assert max((a - b).abs().max().item() for a, b in zip(pa, pb)) <= 1e-6
 
 
-def test_refiner_train_loop_and_checkpoint_interop_emulated(tmp_path):
+def test_refiner_train_loop_and_checkpoint_interop_emulated(tmp_path, monkeypatch):
     """epipolarpose_b200/refiner/main.py train() / test() / save_ckpt (reference refiner/main.py:
     31-84, refiner/utils.py:18-36) through the emulated ABI: parameters after an epoch equal an
     independent loop built from the oracle network + torch.optim.Adam + torch's clip_grad_norm_
@@ -732,6 +732,7 @@ def test_refiner_train_loop_and_checkpoint_interop_emulated(tmp_path):
     from oracle import restate_refiner as rr
     from epipolarpose_b200.refiner import main as rmain, model as rmodel, utils as rutils, data as rdata
     import lib.utils.utils as U
+    monkeypatch.setattr(rmain, "_to_device", lambda t: t)     # the emulation computes on the host
     rmodel.LinearModelPG._backend[0] = emul_ops
     rutils._backend[0] = emul_ops
     U._backend[0] = emul_ops
