@@ -66,20 +66,21 @@ _PROTOS = {
     "epb_patch_sample_occ": (c_int, [c_p] * 7 + [c_int, c_int, c_int] + [c_p] * 5 + [c_p]),
     "epb_patch_joints": (c_int, [c_p, c_p, c_p, c_int, c_int, c_d, c_d, c_d, c_int, c_p, c_p]),
     "epb_bn_finalize_scale": (c_int, [c_p, c_i64, c_int, c_p, c_p, c_f, c_f] + [c_p] * 12),
-    "epb_softargmax_bwd_split": (c_int, [c_p] + [c_int] * 5 + [c_p] * 7),
+    "epb_softargmax_bwd_split": (c_int, [c_p] + [c_int] * 5 + [c_p] * 6 + [c_int, c_p]),
     "epb_act_scale": (c_int, [c_p, c_p, c_p, c_i64, c_int, c_p, c_p, c_p, c_p, c_p, c_p]),
-    "epb_bn_act_split": (c_int, [c_p] * 8 + [c_int, c_i64, c_int, c_p, c_p, c_p, c_p]),
-    "epb_bn_relu_maxpool_split": (c_int, [c_p] * 6 + [c_int] * 4 + [c_p]),
-    "epb_im2col_split": (c_int, [c_p] * 3 + [c_int] * 11 + [c_p]),
-    "epb_split16": (c_int, [c_p, ctypes.c_longlong, c_p, c_p, c_p, c_p]),
-    "epb_split16_batch": (c_int, [c_p, c_int, ctypes.c_longlong, c_p, c_p]),
-    "epb_conv16_fprop": (c_int, [ctypes.POINTER(ConvGeom)] + [c_p] * 8),
-    "epb_conv16_wgrad": (c_int, [ctypes.POINTER(ConvGeom)] + [c_p] * 6 + [ctypes.c_longlong, c_p]),
+    # split-fp16 family: the int before the stream is the plane count (1 or 2)
+    "epb_bn_act_split": (c_int, [c_p] * 8 + [c_int, c_i64, c_int, c_p, c_p, c_p, c_int, c_p]),
+    "epb_bn_relu_maxpool_split": (c_int, [c_p] * 6 + [c_int] * 5 + [c_p]),
+    "epb_im2col_split": (c_int, [c_p] * 3 + [c_int] * 12 + [c_p]),
+    "epb_split16": (c_int, [c_p, ctypes.c_longlong, c_p, c_p, c_p, c_int, c_p]),
+    "epb_split16_batch": (c_int, [c_p, c_int, ctypes.c_longlong, c_p, c_int, c_p]),
+    "epb_conv16_fprop": (c_int, [ctypes.POINTER(ConvGeom)] + [c_p] * 7 + [c_int, c_p]),
+    "epb_conv16_wgrad": (c_int, [ctypes.POINTER(ConvGeom)] + [c_p] * 6 + [ctypes.c_longlong, c_int, c_p]),
     "epb_bn_bwd_reduce_mx": (c_int, [c_p] * 7 + [c_int, c_i64, c_int, c_p, c_p, c_p]),
-    "epb_bn_bwd_apply_split": (c_int, [c_p] * 8 + [c_int, c_p, c_p, c_i64, c_int] + [c_p] * 6),
-    "epb_bn_bwd_split": (c_int, [c_p] * 9 + [c_int, c_i64, c_int] + [c_p] * 6),
+    "epb_bn_bwd_apply_split": (c_int, [c_p] * 8 + [c_int, c_p, c_p, c_i64, c_int] + [c_p] * 5 + [c_int, c_p]),
+    "epb_bn_bwd_split": (c_int, [c_p] * 9 + [c_int, c_i64, c_int] + [c_p] * 5 + [c_int, c_p]),
     "epb_debug_conv16_trace": (c_int, [c_p, c_int]),
-    "epb_avgpool_split": (c_int, [c_p, c_p, c_p, c_int, c_int, c_int, c_p]),
+    "epb_avgpool_split": (c_int, [c_p, c_p, c_p, c_int, c_int, c_int, c_int, c_p]),
     "epb_sumsq": (c_int, [c_p, c_i64, c_p, c_p]),
     "epb_clip_scale": (c_int, [c_p, c_i64, c_p, c_d, c_p]),
     "epb_adam_step": (c_int, [c_p, c_p, c_p, c_p, c_i64, c_f, c_f, c_f, c_f, c_f, c_int, c_f, c_p]),

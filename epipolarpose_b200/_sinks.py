@@ -14,11 +14,14 @@ import torch
 
 
 class LogitGradSink:
-    __slots__ = ("ptr", "shape", "planes", "sc", "dbias", "filled", "token")
+    """nplanes: plane count of the split gradient the network's backward takes (2: hi + lo,
+    1: hi only, the single-pass f16 mode)."""
+    __slots__ = ("ptr", "shape", "nplanes", "planes", "sc", "dbias", "filled", "token")
 
-    def __init__(self, logits_nchw_view):
+    def __init__(self, logits_nchw_view, nplanes=2):
         t = logits_nchw_view
         self.ptr, self.shape = t.data_ptr(), tuple(t.shape)
+        self.nplanes = nplanes
         self.planes = self.sc = self.dbias = None
         self.filled = False
         self.token = torch.zeros(1, device=t.device, dtype=torch.float32)
@@ -28,3 +31,10 @@ class LogitGradSink:
 
     def is_token(self, g):
         return g.data_ptr() == self.token.data_ptr() and all(s == 0 for s in g.stride())
+
+    def dense(self):
+        """The gradient the planes hold, fp32, in their NHWC layout."""
+        g = self.planes[0].float()
+        if self.nplanes == 2:
+            g = g + self.planes[1].float()
+        return g * self.sc[1]

@@ -6,6 +6,9 @@
 //   out[m, co] = (1 / (s_in * s_w)) * sum_k A[m, k] * W[co, k],   m = phase-grid pixel,
 //   k = (tap, ci),  A = hi + lo, W = hi + lo  (fp16 planes),
 //   A*W ~= A_lo*W_hi + A_hi*W_lo + A_hi*W_hi   (three kind::f16 passes, FP32 accumulate).
+// Single-pass ("f16") form, template NP = 1: the operands are the hi planes alone (10 explicit
+// mantissa bits, TF32-class), A*W ~= A_hi*W_hi, one kind::f16 pass per k-step; the smem of the
+// missing lo boxes deepens the operand ring.
 //
 // Both operands are TMA-fed: the activation planes are post-BatchNorm/ReLU (written once by
 // split16.cu), so an M tile of 128 pixels is ONE 5-D box load per plane and tap -- (64 channels,
@@ -16,8 +19,9 @@
 // Always CTA pairs (cluster of 2, tcgen05 cta_group::2, M = 256): each CTA holds its 128 A
 // rows and HALF of the B tile's N rows, which keeps shared-memory reads under 128 B/clk at
 // the kind::f16 rate.  One persistent cluster per SM pair, 6 warps per CTA:
-//   warp 0    TMA producer (one lane): A hi/lo + B hi/lo boxes per k-block, S-deep ring;
-//   warp 1    MMA issuer (leader CTA, one lane): 4 k-steps x 3 tcgen05.mma per k-block,
+//   warp 0    TMA producer (one lane): A hi/lo + B hi/lo boxes (hi only when NP = 1) per
+//             k-block, S-deep ring;
+//   warp 1    MMA issuer (leader CTA, one lane): 4 k-steps x 3 (NP = 1: 1) tcgen05.mma per k-block,
 //             FP32 accumulators double buffered in TMEM;
 //   warps 2-5 epilogue: tcgen05.ld -> scale / bias -> 128B-swizzled smem box -> ONE TMA store
 //             (or TMA reduce-add for the accumulate form) per 32x32 block: no per-row address
@@ -64,31 +68,36 @@ struct Maps16 {
   CUtensorMap o;                 // fp32 output, box = 32 channels x 32 tile rows
 };
 
-template <int BN>
+// NP: operand planes (2: hi + lo, three passes; 1: hi only, one pass)
+template <int BN, int NP>
 struct Cfg16 {
   static constexpr int BROWS = BN / 2;                 // B rows held by this CTA
   static constexpr int A_PLANE = BM * 128;
   static constexpr int B_PLANE = BROWS * 128;
-  static constexpr int A_BYTES = 2 * A_PLANE;
-  static constexpr int B_BYTES = 2 * B_PLANE;
+  static constexpr int A_BYTES = NP * A_PLANE;
+  static constexpr int B_BYTES = NP * B_PLANE;
   static constexpr int STAGE = A_BYTES + B_BYTES;
-  static constexpr int S_ = kStageBudget / STAGE;
-  static constexpr int S = S_ > 6 ? 6 : S_;
   static constexpr int TMEM_COLS = (2 * BN <= 128) ? 128 : (2 * BN <= 256 ? 256 : 512);
   static constexpr int EPI_BYTES = kEpiWarps * 4096;           // one swizzled 32x32 fp32 box per warp
   static constexpr int STAT_BYTES = kEpiWarps * 2 * BN * 4;    // per-warp [sum | sum of squares][BN]
-  static constexpr int SMEM = S * STAGE + EPI_BYTES + 1024 /*align*/ + 1024 /*barriers*/ + STAT_BYTES;
+  static constexpr int FIXED = EPI_BYTES + 1024 /*align*/ + 1024 /*barriers*/ + STAT_BYTES;
+  // two planes: the measured ring (<= 6 stages in 192 KB); one plane: as deep as the 227 KB
+  // allow, up to the 8 full / empty barrier pairs (BN 256: 6, BN 128 / 64: 8 stages)
+  static constexpr int S_ = NP == 2 ? kStageBudget / STAGE : (227 * 1024 - FIXED) / STAGE;
+  static constexpr int S_MAX = NP == 2 ? 6 : 8;
+  static constexpr int S = S_ > S_MAX ? S_MAX : S_;
+  static constexpr int SMEM = S * STAGE + FIXED;
   static_assert(SMEM <= 227 * 1024, "shared memory budget");
   static_assert(S >= 2, "ring too shallow");
 };
 
-template <int BN>
+template <int BN, int NP>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads16, 1)
 conv16_kernel(const __grid_constant__ Plan16 P, const __grid_constant__ Maps16 maps,
               const float* __restrict__ in_sc, const float* __restrict__ w_sc,
               const float* __restrict__ bias, float* __restrict__ out,
               double* __restrict__ stats) {
-  using C = Cfg16<BN>;
+  using C = Cfg16<BN, NP>;
   const int crank = (int)tc::cluster_ctarank();
   const int tile0 = (int)tc::cluster_id_x();
   const int tstep = (int)tc::cluster_count_x();
@@ -161,11 +170,11 @@ conv16_kernel(const __grid_constant__ Plan16 P, const __grid_constant__ Maps16 m
           const CUtensorMap* am = &maps.a[P.map[t]];
           const int cx = cb * 64, wx = w0 + P.dwq[t], hx = h0 + P.dhq[t];
           tc::tma_load_5d_pair(a_dst, am, lead_bar, cx, wx, hx, n0, 0);
-          tc::tma_load_5d_pair(a_dst + C::A_PLANE, am, lead_bar, cx, wx, hx, n0, 1);
+          if (NP == 2) tc::tma_load_5d_pair(a_dst + C::A_PLANE, am, lead_bar, cx, wx, hx, n0, 1);
           const uint32_t b_dst = a_dst + C::A_BYTES;
           const int kx = P.koff[t] + cx, rx = nt * BN + crank * C::BROWS;
           tc::tma_load_3d_pair(b_dst, &maps.w, lead_bar, kx, rx, 0);
-          tc::tma_load_3d_pair(b_dst + C::B_PLANE, &maps.w, lead_bar, kx, rx, 1);
+          if (NP == 2) tc::tma_load_3d_pair(b_dst + C::B_PLANE, &maps.w, lead_bar, kx, rx, 1);
           if (++cb == P.CB) { cb = 0; ++t; }
           if (++stage == C::S) { stage = 0; phase ^= 1; }
         }
@@ -192,12 +201,16 @@ conv16_kernel(const __grid_constant__ Plan16 P, const __grid_constant__ Maps16 m
 #pragma unroll
           for (int kk = 0; kk < 4; ++kk) {               // 4 x K = 16 fp16 (32 bytes)
             const uint64_t ah = tc::desc_kmajor_sw128(a_hi + kk * 32);
-            const uint64_t al = tc::desc_kmajor_sw128(a_hi + C::A_PLANE + kk * 32);
             const uint64_t bh = tc::desc_kmajor_sw128(b_hi + kk * 32);
-            const uint64_t bl = tc::desc_kmajor_sw128(b_hi + C::B_PLANE + kk * 32);
-            tc::mma_f16_pair(d_tmem, al, bh, idesc, (kb | kk) != 0);
-            tc::mma_f16_pair(d_tmem, ah, bl, idesc, 1);
-            tc::mma_f16_pair(d_tmem, ah, bh, idesc, 1);
+            if (NP == 2) {
+              const uint64_t al = tc::desc_kmajor_sw128(a_hi + C::A_PLANE + kk * 32);
+              const uint64_t bl = tc::desc_kmajor_sw128(b_hi + C::B_PLANE + kk * 32);
+              tc::mma_f16_pair(d_tmem, al, bh, idesc, (kb | kk) != 0);
+              tc::mma_f16_pair(d_tmem, ah, bl, idesc, 1);
+              tc::mma_f16_pair(d_tmem, ah, bh, idesc, 1);
+            } else {
+              tc::mma_f16_pair(d_tmem, ah, bh, idesc, (kb | kk) != 0);
+            }
           }
           tc::mma_commit_pair(empty_bar(stage));          // frees the slot in both CTAs
           if (++stage == C::S) { stage = 0; phase ^= 1; }
@@ -349,19 +362,19 @@ conv16_kernel(const __grid_constant__ Plan16 P, const __grid_constant__ Maps16 m
   }
 }
 
-template <int BN>
+template <int BN, int NP>
 int launch16(const Plan16& P, const Maps16& maps, const float* in_sc, const float* w_sc,
              const float* bias, float* out, double* stats, cudaStream_t st) {
-  using C = Cfg16<BN>;
+  using C = Cfg16<BN, NP>;
   static bool attr_set = false;
   if (!attr_set) {
-    EPB_CUDA(cudaFuncSetAttribute(conv16_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    EPB_CUDA(cudaFuncSetAttribute(conv16_kernel<BN, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   C::SMEM));
     attr_set = true;
   }
   const int64_t pairs = (int64_t)((P.m_tiles + 1) / 2) * P.n_tiles;
   const int grid = 2 * (int)(pairs < kNumSMs / 2 ? pairs : kNumSMs / 2);
-  conv16_kernel<BN><<<grid, kThreads16, C::SMEM, st>>>(P, maps, in_sc, w_sc, bias, out, stats);
+  conv16_kernel<BN, NP><<<grid, kThreads16, C::SMEM, st>>>(P, maps, in_sc, w_sc, bias, out, stats);
   EPB_LAUNCH_CHECK();
   return EPB_OK;
 }
@@ -378,10 +391,12 @@ extern "C" __attribute__((visibility("default"))) int epb_debug_conv16_trace(lon
 
 extern "C" __attribute__((visibility("default"))) int epb_conv16_fprop(
     const epb_conv_geom* g, const epb_half* in, const float* in_sc, const epb_half* w,
-    const float* w_sc, const float* bias, float* out, double* stats, epb_stream_t stream) {
+    const float* w_sc, const float* bias, float* out, double* stats, int planes,
+    epb_stream_t stream) {
   int rc = epb_conv_geom_check(g);
   if (rc) return rc;
   EPB_CHECK_ARG(in && in_sc && w && w_sc && out);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   EPB_CHECK_ARG(g->Cin % 64 == 0 && g->Cout % 4 == 0 && g->Cout >= 4);
   EPB_CHECK_ARG(g->is == 1 || g->is == 2);
   EPB_CHECK_ARG(!(stats && g->accumulate));
@@ -422,7 +437,8 @@ extern "C" __attribute__((visibility("default"))) int epb_conv16_fprop(
   }
   for (int v = 0; v < 4; ++v) {
     if (!need[v]) continue;
-    rc = epb_make_act_map(&maps.a[v], in, N, Hi, Wi, g->Cin, g->is, v >> 1, v & 1, P.tw, P.th, P.tn);
+    rc = epb_make_act_map(&maps.a[v], in, N, Hi, Wi, g->Cin, g->is, v >> 1, v & 1, P.tw, P.th, P.tn,
+                          planes);
     if (rc) return rc;
   }
   for (int v = 0; v < 4; ++v)
@@ -483,7 +499,7 @@ extern "C" __attribute__((visibility("default"))) int epb_conv16_fprop(
       return EPB_ECUDA;
     }
     const int64_t K = (int64_t)g->Tw * g->Cin;
-    const cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)g->Cout, 2};
+    const cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)g->Cout, (cuuint64_t)planes};
     const cuuint64_t strides[2] = {(cuuint64_t)K * 2, (cuuint64_t)K * 2 * g->Cout};
     const cuuint32_t box[3] = {64, (cuuint32_t)(bn / 2), 1};
     const cuuint32_t estr[3] = {1, 1, 1};
@@ -497,7 +513,12 @@ extern "C" __attribute__((visibility("default"))) int epb_conv16_fprop(
     }
   }
   cudaStream_t st = as_stream(stream);
-  if (bn == 64) return launch16<64>(P, maps, in_sc, w_sc, bias, out, stats, st);
-  if (bn == 128) return launch16<128>(P, maps, in_sc, w_sc, bias, out, stats, st);
-  return launch16<256>(P, maps, in_sc, w_sc, bias, out, stats, st);
+  if (planes == 1) {
+    if (bn == 64) return launch16<64, 1>(P, maps, in_sc, w_sc, bias, out, stats, st);
+    if (bn == 128) return launch16<128, 1>(P, maps, in_sc, w_sc, bias, out, stats, st);
+    return launch16<256, 1>(P, maps, in_sc, w_sc, bias, out, stats, st);
+  }
+  if (bn == 64) return launch16<64, 2>(P, maps, in_sc, w_sc, bias, out, stats, st);
+  if (bn == 128) return launch16<128, 2>(P, maps, in_sc, w_sc, bias, out, stats, st);
+  return launch16<256, 2>(P, maps, in_sc, w_sc, bias, out, stats, st);
 }

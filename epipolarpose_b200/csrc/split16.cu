@@ -5,6 +5,9 @@
 // autograd.  Every kernel is one HBM pass: fp32 rows in, two fp16 planes out (the same
 // 4 bytes per element as an fp32 store), so that the tensor-core kernels (conv16.cu,
 // wgrad16.cu) can take their operands by TMA with no transformation.
+// `planes` (1 or 2) is the plane count of the split tensors a kernel writes or reads: with 1
+// (the single-pass "f16" mode) only the hi plane exists, [1][rows][C], and nothing is written
+// where the lo plane would lie; the hi plane is the same either way.
 #include <cuda_fp16.h>
 #include "common.cuh"
 
@@ -69,7 +72,7 @@ bn_act_split_kernel(const float* __restrict__ x, const float* __restrict__ scale
                     const float* __restrict__ rscale, const float* __restrict__ rshift,
                     const uint4* __restrict__ rs, const float* __restrict__ rs_sc, int relu,
                     int64_t total8, int C8, uint4* __restrict__ y, const float* __restrict__ y_sc,
-                    uint8_t* __restrict__ mask_bits) {
+                    uint8_t* __restrict__ mask_bits, int planes) {
   const float s = y_sc[0];
   const float rinv = rs ? rs_sc[1] : 0.f;
   for (int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x; i < total8;
@@ -98,7 +101,7 @@ bn_act_split_kernel(const float* __restrict__ x, const float* __restrict__ scale
       for (int k = 0; k < 8; ++k) v[k] += q[k];
     } else if (rs) {
       float q[8];
-      join8(rs[i], rs[total8 + i], rinv, q);
+      join8(rs[i], planes == 2 ? rs[total8 + i] : make_uint4(0u, 0u, 0u, 0u), rinv, q);
 #pragma unroll
       for (int k = 0; k < 8; ++k) v[k] += q[k];
     }
@@ -115,7 +118,7 @@ bn_act_split_kernel(const float* __restrict__ x, const float* __restrict__ scale
     uint4 hi, lo;
     split8(v, s, hi, lo);
     y[i] = hi;
-    y[total8 + i] = lo;
+    if (planes == 2) y[total8 + i] = lo;
   }
 }
 
@@ -123,7 +126,7 @@ __global__ void __launch_bounds__(kThreads)
 bn_relu_maxpool_split_kernel(const float* __restrict__ x, const float* __restrict__ scale,
                              const float* __restrict__ shift, uint4* __restrict__ y,
                              const float* __restrict__ y_sc, uint2* __restrict__ argidx, int N, int H,
-                             int W, int C8) {
+                             int W, int C8, int planes) {
   const int Ho = (H + 2 - 3) / 2 + 1, Wo = (W + 2 - 3) / 2 + 1;
   const int64_t total = (int64_t)N * Ho * Wo * C8;
   const float s = y_sc[0];
@@ -161,7 +164,7 @@ bn_relu_maxpool_split_kernel(const float* __restrict__ x, const float* __restric
     uint4 hi, lo;
     split8(best, s, hi, lo);
     y[i] = hi;
-    y[total + i] = lo;
+    if (planes == 2) y[total + i] = lo;
     if (argidx) {
       uint2 a;
       a.x = bi[0] | (bi[1] << 8) | (bi[2] << 16) | ((unsigned)bi[3] << 24);
@@ -176,7 +179,7 @@ bn_relu_maxpool_split_kernel(const float* __restrict__ x, const float* __restric
 __global__ void __launch_bounds__(kThreads)
 im2col_split_kernel(const float* __restrict__ img, uint4* __restrict__ col,
                     const float* __restrict__ col_sc, int N, int C, int Hi, int Wi, int kh, int kw,
-                    int stride, int pad, int Ho, int Wo, int Kpad) {
+                    int stride, int pad, int Ho, int Wo, int Kpad, int planes) {
   extern __shared__ int lut[];                 // [Kpad]: (c*Hi + r)*Wi + s | r << 24 ... packed below
   int* off = lut;                              // element offset of (c, r, s) relative to (ih0, iw0)
   int* rs = lut + Kpad;                        // r << 16 | s ; -1 for padding columns
@@ -216,7 +219,7 @@ im2col_split_kernel(const float* __restrict__ img, uint4* __restrict__ col,
     uint4 hi, lo;
     split8(v, s, hi, lo);
     col[i] = hi;
-    col[total + i] = lo;
+    if (planes == 2) col[total + i] = lo;
   }
 }
 
@@ -228,7 +231,7 @@ constexpr int kSeg = 64;
 __global__ void __launch_bounds__(kThreads)
 im2col_split_tiled_kernel(const float* __restrict__ img, uint4* __restrict__ col,
                           const float* __restrict__ col_sc, int N, int C, int Hi, int Wi, int kh, int kw,
-                          int stride, int pad, int Ho, int Wo, int Kpad, int segs, int tw) {
+                          int stride, int pad, int Ho, int Wo, int Kpad, int segs, int tw, int planes) {
   extern __shared__ int smi[];
   int* lut = smi;                               // [8][Kpad/8]: window offset of (c, r, s), -1 for padding columns
   float* win = reinterpret_cast<float*>(smi + Kpad);        // [C][kh][tw]
@@ -275,7 +278,7 @@ im2col_split_tiled_kernel(const float* __restrict__ img, uint4* __restrict__ col
     uint4 hi, lo;
     split8(v, s, hi, lo);
     col[row0 + it] = hi;
-    col[total + row0 + it] = lo;
+    if (planes == 2) col[total + row0 + it] = lo;
   }
 }
 
@@ -322,7 +325,7 @@ __device__ __forceinline__ float pow2_scale(float amax) {
 
 __global__ void __launch_bounds__(kThreads)
 split_apply_kernel(const epb_split_job* __restrict__ jobs, int njobs,
-                   const uint32_t* __restrict__ amax) {
+                   const uint32_t* __restrict__ amax, int planes) {
   int ji;
   const epb_split_job j = find_job(jobs, njobs, ji);
   const float s = pow2_scale(__uint_as_float(amax[ji]));
@@ -338,7 +341,7 @@ split_apply_kernel(const epb_split_job* __restrict__ jobs, int njobs,
     const float v = j.src[i] * s;
     const __half h = __float2half_rn(v);
     hi[i] = h;
-    lo[i] = __float2half_rn(v - __half2float(h));
+    if (planes == 2) lo[i] = __float2half_rn(v - __half2float(h));
   }
 }
 
@@ -363,7 +366,7 @@ split_amax_one_kernel(const float4* __restrict__ src, int64_t n4, uint32_t* __re
 
 __global__ void __launch_bounds__(kThreads)
 split_apply_one_kernel(const float4* __restrict__ src, int64_t n4, const uint32_t* __restrict__ amax,
-                       uint2* __restrict__ dst, float* __restrict__ sc) {
+                       uint2* __restrict__ dst, float* __restrict__ sc, int planes) {
   const float s = pow2_scale(__uint_as_float(*amax));
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     sc[0] = s;
@@ -375,7 +378,7 @@ split_apply_one_kernel(const float4* __restrict__ src, int64_t n4, const uint32_
     split2(v.x, v.y, s, hi.x, lo.x);
     split2(v.z, v.w, s, hi.y, lo.y);
     dst[i] = hi;
-    dst[n4 + i] = lo;
+    if (planes == 2) dst[n4 + i] = lo;
   }
 }
 
@@ -625,7 +628,7 @@ bn_bwd_apply_split_kernel(const float4* dy /* may alias dy_masked */, const floa
                           int relu, const float4* __restrict__ k1v, const float4* __restrict__ k2v,
                           uint2* __restrict__ dz, float* __restrict__ dz_sc,
                           const float* __restrict__ bound, float4* dy_masked, int64_t total4, int C4,
-                          int mask_bits) {
+                          int mask_bits, int planes) {
   // scale of dz: from the bound the combine pass left (fused entry point), else as published in dz_sc
   const float s = bound ? pow2_scale(*bound) : dz_sc[0];
   if (bound && blockIdx.x == 0 && threadIdx.x == 0) {
@@ -676,7 +679,7 @@ bn_bwd_apply_split_kernel(const float4* dy /* may alias dy_masked */, const floa
       split2(o.x, o.y, s, hi.x, lo.x);
       split2(o.z, o.w, s, hi.y, lo.y);
       dz[i] = hi;
-      dz[total4 + i] = lo;
+      if (planes == 2) dz[total4 + i] = lo;
       if (dy_masked) dy_masked[i] = g;
     }
   }
@@ -804,7 +807,7 @@ __global__ void softargmax_bwd_split_kernel(const float* __restrict__ logits, in
                                             const float* __restrict__ lse,
                                             const float* __restrict__ dcoords,
                                             const float* __restrict__ sc, uint2* __restrict__ planes,
-                                            int64_t total4, float* __restrict__ parts) {
+                                            int64_t total4, float* __restrict__ parts, int nplanes) {
   extern __shared__ float4 shq[];            // [blockDim]
   const int n = blockIdx.y, sp = blockIdx.x;
   const int C4 = (J * D) >> 2;
@@ -839,7 +842,7 @@ __global__ void softargmax_bwd_split_kernel(const float* __restrict__ logits, in
     split2(o.z, o.w, s, hi.y, lo.y);
     const int64_t i = img + (int64_t)pix * C4;
     planes[i] = hi;
-    planes[total4 + i] = lo;
+    if (nplanes == 2) planes[total4 + i] = lo;
     acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w;
     x += ppi;
     while (x >= W) { x -= W; ++y; }
@@ -885,14 +888,14 @@ colsum_parts_kernel(const float* __restrict__ parts, int rows, int C, float* __r
 }
 
 __global__ void avgpool_split_kernel(const __half* __restrict__ x, const float* __restrict__ x_sc,
-                                     float* __restrict__ y, int N, int HW, int C) {
+                                     float* __restrict__ y, int N, int HW, int C, int planes) {
   const int n = blockIdx.y, c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
   const int64_t plane = (int64_t)N * HW * C;
   float acc = 0.f;
   for (int p = 0; p < HW; ++p) {
     const int64_t i = ((int64_t)n * HW + p) * C + c;
-    acc += __half2float(x[i]) + __half2float(x[plane + i]);
+    acc += planes == 2 ? __half2float(x[i]) + __half2float(x[plane + i]) : __half2float(x[i]);
   }
   y[(int64_t)n * C + c] = acc * x_sc[1] / (float)HW;
 }
@@ -904,8 +907,9 @@ __global__ void avgpool_split_kernel(const __half* __restrict__ x, const float* 
 EPB_API int epb_bn_act_split(const float* x, const float* scale, const float* shift, const float* r,
                              const float* rscale, const float* rshift, const epb_half* r_split,
                              const float* r_sc, int relu, int64_t M, int C, epb_half* y,
-                             const float* y_sc, uint8_t* mask_bits, epb_stream_t stream) {
+                             const float* y_sc, uint8_t* mask_bits, int planes, epb_stream_t stream) {
   EPB_CHECK_ARG(x && y && y_sc && M > 0 && C > 0 && C % 8 == 0);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   EPB_CHECK_ARG((scale == nullptr) == (shift == nullptr));
   EPB_CHECK_ARG((rscale == nullptr) == (rshift == nullptr));
   EPB_CHECK_ARG(!(r && r_split) && ((r_split == nullptr) == (r_sc == nullptr)));
@@ -913,28 +917,30 @@ EPB_API int epb_bn_act_split(const float* x, const float* scale, const float* sh
   const int64_t total8 = M * (C / 8);
   bn_act_split_kernel<<<ew_blocks(total8), kThreads, 0, as_stream(stream)>>>(
       x, scale, shift, r, rscale, rshift, reinterpret_cast<const uint4*>(r_split), r_sc, relu, total8,
-      C / 8, reinterpret_cast<uint4*>(y), y_sc, mask_bits);
+      C / 8, reinterpret_cast<uint4*>(y), y_sc, mask_bits, planes);
   EPB_LAUNCH_CHECK();
   return EPB_OK;
 }
 
 EPB_API int epb_bn_relu_maxpool_split(const float* x, const float* scale, const float* shift,
                                       epb_half* y, const float* y_sc, uint8_t* argidx, int N, int H,
-                                      int W, int C, epb_stream_t stream) {
+                                      int W, int C, int planes, epb_stream_t stream) {
   EPB_CHECK_ARG(x && scale && shift && y && y_sc && N > 0 && H > 0 && W > 0 && C > 0 && C % 8 == 0);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   const int Ho = (H + 2 - 3) / 2 + 1, Wo = (W + 2 - 3) / 2 + 1;
   const int64_t total = (int64_t)N * Ho * Wo * (C / 8);
   bn_relu_maxpool_split_kernel<<<ew_blocks(total), kThreads, 0, as_stream(stream)>>>(
       x, scale, shift, reinterpret_cast<uint4*>(y), y_sc, reinterpret_cast<uint2*>(argidx), N, H, W,
-      C / 8);
+      C / 8, planes);
   EPB_LAUNCH_CHECK();
   return EPB_OK;
 }
 
 EPB_API int epb_im2col_split(const float* img_nchw, epb_half* col, const float* col_sc, int N, int C,
                              int Hi, int Wi, int kh, int kw, int stride, int pad, int Ho, int Wo,
-                             int Kpad, epb_stream_t stream) {
+                             int Kpad, int planes, epb_stream_t stream) {
   EPB_CHECK_ARG(img_nchw && col && col_sc && N > 0 && C > 0 && Kpad % 8 == 0 && Kpad >= kh * kw * C);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   const int64_t total = (int64_t)N * Ho * Wo * (Kpad / 8);
   EPB_CHECK_ARG(Kpad <= 4096);
   {
@@ -944,25 +950,27 @@ EPB_API int epb_im2col_split(const float* img_nchw, epb_half* col, const float* 
     if (smem <= 48 * 1024 && ctas < (1LL << 31)) {
       im2col_split_tiled_kernel<<<(unsigned)ctas, kThreads, smem, as_stream(stream)>>>(
           img_nchw, reinterpret_cast<uint4*>(col), col_sc, N, C, Hi, Wi, kh, kw, stride, pad, Ho, Wo, Kpad,
-          segs, tw);
+          segs, tw, planes);
       EPB_LAUNCH_CHECK();
       return EPB_OK;
     }
   }
   im2col_split_kernel<<<ew_blocks(total), kThreads, 2 * Kpad * sizeof(int), as_stream(stream)>>>(
-      img_nchw, reinterpret_cast<uint4*>(col), col_sc, N, C, Hi, Wi, kh, kw, stride, pad, Ho, Wo, Kpad);
+      img_nchw, reinterpret_cast<uint4*>(col), col_sc, N, C, Hi, Wi, kh, kw, stride, pad, Ho, Wo, Kpad,
+      planes);
   EPB_LAUNCH_CHECK();
   return EPB_OK;
 }
 
 EPB_API int epb_split16_batch(const epb_split_job* jobs, int njobs, long long total_blocks,
-                              uint32_t* amax_ws, epb_stream_t stream) {
+                              uint32_t* amax_ws, int planes, epb_stream_t stream) {
   EPB_CHECK_ARG(jobs && amax_ws && njobs > 0 && total_blocks > 0 && total_blocks < (1LL << 31));
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   cudaStream_t st = as_stream(stream);
   EPB_CUDA(cudaMemsetAsync(amax_ws, 0, sizeof(uint32_t) * njobs, st));
   split_amax_kernel<<<(unsigned)total_blocks, kThreads, 0, st>>>(jobs, njobs, amax_ws);
   EPB_LAUNCH_CHECK();
-  split_apply_kernel<<<(unsigned)total_blocks, kThreads, 0, st>>>(jobs, njobs, amax_ws);
+  split_apply_kernel<<<(unsigned)total_blocks, kThreads, 0, st>>>(jobs, njobs, amax_ws, planes);
   EPB_LAUNCH_CHECK();
   return EPB_OK;
 }
@@ -1028,8 +1036,9 @@ EPB_API int epb_bn_bwd_split(const float* dy, const float* x, const epb_half* ma
                              const uint8_t* mask_bits, const float* scale, const float* shift, const float* mean,
                              const float* invstd, const float* gamma, int relu, int64_t M, int C,
                              epb_half* dz, float* dz_sc, float* dy_masked, float* dgamma,
-                             float* dbeta, epb_stream_t stream) {
+                             float* dbeta, int planes, epb_stream_t stream) {
   EPB_CHECK_ARG(dy && x && scale && shift && mean && invstd && dz && dz_sc);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   EPB_CHECK_ARG(M > 0 && C > 0 && C % 4 == 0);
   EPB_CHECK_ARG(!(mask_hi && mask_bits) && (!mask_bits || C % 8 == 0));
   const int mask_kind = mask_bits ? 2 : 1;
@@ -1055,7 +1064,7 @@ EPB_API int epb_bn_bwd_split(const float* dy, const float* x, const epb_half* ma
       reinterpret_cast<const float4*>(invstd), reinterpret_cast<const float4*>(gamma), relu,
       reinterpret_cast<const float4*>(coef), reinterpret_cast<const float4*>(coef + C),
       reinterpret_cast<uint2*>(dz), dz_sc, reinterpret_cast<const float*>(bound),
-      reinterpret_cast<float4*>(dy_masked), total4, C / 4, mask_kind == 2);
+      reinterpret_cast<float4*>(dy_masked), total4, C / 4, mask_kind == 2, planes);
   EPB_LAUNCH_CHECK();
   return EPB_OK;
 }
@@ -1065,8 +1074,9 @@ EPB_API int epb_bn_bwd_apply_split(const float* dy, const float* x, const epb_ha
                                    const float* invstd, const float* gamma, int relu,
                                    const double* sums, const float* maxes, int64_t M, int C,
                                    epb_half* dz, float* dz_sc, float* dy_masked, float* dgamma,
-                                   float* dbeta, epb_stream_t stream) {
+                                   float* dbeta, int planes, epb_stream_t stream) {
   EPB_CHECK_ARG(dy && x && scale && shift && mean && invstd && sums && maxes && dz && dz_sc);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   EPB_CHECK_ARG(M > 0 && C > 0 && C % 4 == 0);
   cudaStream_t st = as_stream(stream);
   float* mx = const_cast<float*>(maxes);      // consumed here: overwritten by the coefficients
@@ -1080,16 +1090,18 @@ EPB_API int epb_bn_bwd_apply_split(const float* dy, const float* x, const epb_ha
       reinterpret_cast<const float4*>(shift), reinterpret_cast<const float4*>(mean),
       reinterpret_cast<const float4*>(invstd), reinterpret_cast<const float4*>(gamma), relu,
       reinterpret_cast<const float4*>(mx), reinterpret_cast<const float4*>(mx + C),
-      reinterpret_cast<uint2*>(dz), dz_sc, nullptr, reinterpret_cast<float4*>(dy_masked), total4, C / 4, 0);
+      reinterpret_cast<uint2*>(dz), dz_sc, nullptr, reinterpret_cast<float4*>(dy_masked), total4, C / 4, 0,
+      planes);
   EPB_LAUNCH_CHECK();
   return EPB_OK;
 }
 
 EPB_API int epb_avgpool_split(const epb_half* x, const float* x_sc, float* y, int N, int HW, int C,
-                              epb_stream_t stream) {
+                              int planes, epb_stream_t stream) {
   EPB_CHECK_ARG(x && x_sc && y && N > 0 && HW > 0 && C > 0);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   avgpool_split_kernel<<<dim3((C + 127) / 128, N), 128, 0, as_stream(stream)>>>(
-      reinterpret_cast<const __half*>(x), x_sc, y, N, HW, C);
+      reinterpret_cast<const __half*>(x), x_sc, y, N, HW, C, planes);
   EPB_LAUNCH_CHECK();
   return EPB_OK;
 }
@@ -1123,8 +1135,10 @@ EPB_API int epb_bn_finalize_scale(const double* stats, int64_t M, int C, const f
 
 EPB_API int epb_softargmax_bwd_split(const float* logits, int N, int J, int D, int H, int W,
                                      const float* coords, const float* lse_ws, const float* dcoords,
-                                     epb_half* dlogits16, float* sc, float* dbias, epb_stream_t stream) {
+                                     epb_half* dlogits16, float* sc, float* dbias, int planes,
+                                     epb_stream_t stream) {
   EPB_CHECK_ARG(logits && coords && lse_ws && dcoords && dlogits16 && sc);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   EPB_CHECK_ARG(N > 0 && J > 0 && D > 0 && H > 0 && W > 0 && D % 4 == 0);
   const int C4 = J * D / 4;
   EPB_CHECK_ARG(C4 <= 1024);
@@ -1140,7 +1154,7 @@ EPB_API int epb_softargmax_bwd_split(const float* logits, int N, int J, int D, i
   const int threads = C4 * ppi;
   softargmax_bwd_split_kernel<<<dim3(S, N), threads, threads * sizeof(float4), st>>>(
       logits, J, D, H, W, S, ppi, coords, lse_ws, dcoords, sc, reinterpret_cast<uint2*>(dlogits16),
-      (int64_t)N * H * W * C4, static_cast<float*>(parts));
+      (int64_t)N * H * W * C4, static_cast<float*>(parts), planes);
   EPB_LAUNCH_CHECK();
   if (dbias) {
     colsum_parts_kernel<<<(C4 * 4 + 7) / 8, 256, 0, st>>>(static_cast<const float*>(parts), N * S,
@@ -1151,8 +1165,9 @@ EPB_API int epb_softargmax_bwd_split(const float* logits, int N, int J, int D, i
 }
 
 EPB_API int epb_split16(const float* src, long long n, epb_half* dst, float* sc, uint32_t* amax_ws,
-                        epb_stream_t stream) {
+                        int planes, epb_stream_t stream) {
   EPB_CHECK_ARG(src && dst && sc && amax_ws && n > 0 && n % 4 == 0);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   cudaStream_t st = as_stream(stream);
   EPB_CUDA(cudaMemsetAsync(amax_ws, 0, sizeof(uint32_t), st));
   const int64_t n4 = n / 4;
@@ -1160,7 +1175,7 @@ EPB_API int epb_split16(const float* src, long long n, epb_half* dst, float* sc,
                                                             amax_ws);
   EPB_LAUNCH_CHECK();
   split_apply_one_kernel<<<ew_blocks(n4), kThreads, 0, st>>>(reinterpret_cast<const float4*>(src), n4,
-                                                             amax_ws, reinterpret_cast<uint2*>(dst), sc);
+                                                             amax_ws, reinterpret_cast<uint2*>(dst), sc, planes);
   EPB_LAUNCH_CHECK();
   return EPB_OK;
 }

@@ -19,11 +19,12 @@ inline void epb_choose_tile(int N, int Hp, int Wp, int rows, int& tw, int& th, i
   }
 }
 
-// 5-D map over the planes of a split NHWC tensor [2][N][H][W][C] fp16, viewed with spatial
-// stride `stride` starting at pixel (qh, qw): coordinates (c, w', h', n, plane) address pixel
-// (h'*stride + qh, w'*stride + qw).  Out-of-range coordinates (negative included) read 0.
+// 5-D map over the planes of a split NHWC tensor [planes][N][H][W][C] fp16 (planes 2: hi, lo;
+// 1: hi only), viewed with spatial stride `stride` starting at pixel (qh, qw): coordinates
+// (c, w', h', n, plane) address pixel (h'*stride + qh, w'*stride + qw).  Out-of-range
+// coordinates (negative included) read 0.
 inline int epb_make_act_map(CUtensorMap* m, const epb_half* base, int N, int H, int W, int C,
-                            int stride, int qh, int qw, int tw, int th, int tn) {
+                            int stride, int qh, int qw, int tw, int th, int tn, int planes) {
   epb_encode_tiled_fn enc = epb_get_encode_tiled();
   if (!enc) {
     epb_set_error("cuTensorMapEncodeTiled entry point unavailable");
@@ -34,7 +35,7 @@ inline int epb_make_act_map(CUtensorMap* m, const epb_half* base, int N, int H, 
     epb_set_error("empty strided view");
     return EPB_EINVAL;
   }
-  const cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)Wv, (cuuint64_t)Hv, (cuuint64_t)N, 2};
+  const cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)Wv, (cuuint64_t)Hv, (cuuint64_t)N, (cuuint64_t)planes};
   const cuuint64_t strides[4] = {(cuuint64_t)stride * C * 2, (cuuint64_t)stride * W * C * 2,
                                  (cuuint64_t)H * W * C * 2, (cuuint64_t)N * H * W * C * 2};
   const cuuint32_t box[5] = {64, (cuuint32_t)tw, (cuuint32_t)th, (cuuint32_t)tn, 1};

@@ -14,6 +14,8 @@
 // layer still fills the M rows; the N side is min(Cout, 256) output channels, half per CTA.
 // The pixel range is split across clusters; partial tiles go to `ws` and are summed in split
 // order by a second kernel (deterministic; no atomics).
+// Template NP = 1 is the single-pass ("f16") form: hi planes only, one tcgen05.mma per k-step,
+// a deeper ring in the smem the lo boxes no longer take.
 #include "split16_common.cuh"
 
 namespace {
@@ -41,23 +43,28 @@ struct MapsW16 {
   CUtensorMap d;
 };
 
-template <int BN>
+// NP: operand planes (2: hi + lo, three passes; 1: hi only, one pass)
+template <int BN, int NP>
 struct CfgW16 {
   static constexpr int BCH = BN / 128;                   // 64-channel chunks of dout per CTA
   static constexpr int A_PLANE = 2 * kChunk;
   static constexpr int B_PLANE = BCH * kChunk;
-  static constexpr int STAGE = 2 * A_PLANE + 2 * B_PLANE;
-  static constexpr int S_ = (192 * 1024) / STAGE;
-  static constexpr int S = S_ > 6 ? 6 : S_;
+  static constexpr int STAGE = NP * A_PLANE + NP * B_PLANE;
+  // two planes: the measured ring (<= 6 stages in 192 KB); one plane: as deep as the 227 KB
+  // allow, up to the 8 full / empty barrier pairs (BN 256: 7, BN 128: 8 stages)
+  static constexpr int S_ = NP == 2 ? (192 * 1024) / STAGE : (227 * 1024 - 1024 - 256) / STAGE;
+  static constexpr int S_MAX = NP == 2 ? 6 : 8;
+  static constexpr int S = S_ > S_MAX ? S_MAX : S_;
   static constexpr int SMEM = S * STAGE + 1024 + 256;
+  static_assert(SMEM <= 227 * 1024, "shared memory budget");
 };
 
-template <int BN>
+template <int BN, int NP>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsW16, 1)
 wgrad16_kernel(const __grid_constant__ PlanW16 P, const __grid_constant__ MapsW16 maps,
                const float* __restrict__ in_sc, const float* __restrict__ dout_sc,
                float* __restrict__ dw, float* __restrict__ ws) {
-  using C = CfgW16<BN>;
+  using C = CfgW16<BN, NP>;
   const int crank = (int)tc::cluster_ctarank();
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = tc::smem_u32(smem_raw);
@@ -119,9 +126,9 @@ wgrad16_kernel(const __grid_constant__ PlanW16 P, const __grid_constant__ MapsW1
         if (crank == 0) tc::mbar_arrive_expect_tx(full_bar(stage), 2 * C::STAGE);
         const uint32_t lead_bar = tc::mapa(full_bar(stage), 0);
         const uint32_t a_dst = base + stage * C::STAGE;
-        const uint32_t b_dst = a_dst + 2 * C::A_PLANE;
+        const uint32_t b_dst = a_dst + NP * C::A_PLANE;
 #pragma unroll
-        for (int pl = 0; pl < 2; ++pl) {
+        for (int pl = 0; pl < NP; ++pl) {
 #pragma unroll
           for (int j = 0; j < 2; ++j) {
             const int t = ct[j];
@@ -146,16 +153,20 @@ wgrad16_kernel(const __grid_constant__ PlanW16 P, const __grid_constant__ MapsW1
         tc::mbar_wait_cluster(full_bar(stage), phase);
         tc::tc_fence_after();
         const uint32_t a_hi = base + stage * C::STAGE;
-        const uint32_t b_hi = a_hi + 2 * C::A_PLANE;
+        const uint32_t b_hi = a_hi + NP * C::A_PLANE;
 #pragma unroll
         for (int ks = 0; ks < KT / 16; ++ks) {
           const uint64_t ah = tc::desc_mnmajor16_sw128(a_hi + ks * 2048, kChunk, 1024);
-          const uint64_t al = tc::desc_mnmajor16_sw128(a_hi + C::A_PLANE + ks * 2048, kChunk, 1024);
           const uint64_t bh = tc::desc_mnmajor16_sw128(b_hi + ks * 2048, kChunk, 1024);
-          const uint64_t bl = tc::desc_mnmajor16_sw128(b_hi + C::B_PLANE + ks * 2048, kChunk, 1024);
-          tc::mma_f16_pair(tmem_base, al, bh, idesc, (k | ks) != 0);
-          tc::mma_f16_pair(tmem_base, ah, bl, idesc, 1);
-          tc::mma_f16_pair(tmem_base, ah, bh, idesc, 1);
+          if (NP == 2) {
+            const uint64_t al = tc::desc_mnmajor16_sw128(a_hi + C::A_PLANE + ks * 2048, kChunk, 1024);
+            const uint64_t bl = tc::desc_mnmajor16_sw128(b_hi + C::B_PLANE + ks * 2048, kChunk, 1024);
+            tc::mma_f16_pair(tmem_base, al, bh, idesc, (k | ks) != 0);
+            tc::mma_f16_pair(tmem_base, ah, bl, idesc, 1);
+            tc::mma_f16_pair(tmem_base, ah, bh, idesc, 1);
+          } else {
+            tc::mma_f16_pair(tmem_base, ah, bh, idesc, (k | ks) != 0);
+          }
         }
         tc::mma_commit_pair(empty_bar(stage));
         if (++stage == C::S) { stage = 0; phase ^= 1; }
@@ -239,19 +250,19 @@ wgrad16_reduce_kernel(const __grid_constant__ PlanW16 P, const float* __restrict
   }
 }
 
-template <int BN>
+template <int BN, int NP>
 int launch_w16(const PlanW16& P, const MapsW16& maps, const float* in_sc, const float* dout_sc,
                float* dw, float* ws, cudaStream_t st) {
-  using C = CfgW16<BN>;
+  using C = CfgW16<BN, NP>;
   static bool attr_set = false;
   if (!attr_set) {
-    EPB_CUDA(cudaFuncSetAttribute(wgrad16_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    EPB_CUDA(cudaFuncSetAttribute(wgrad16_kernel<BN, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   C::SMEM));
     attr_set = true;
   }
   const int64_t clusters = (int64_t)P.groups * P.n_tiles * P.splits;
   EPB_CHECK_ARG(clusters < (1LL << 30));
-  wgrad16_kernel<BN><<<(unsigned)(2 * clusters), kThreadsW16, C::SMEM, st>>>(P, maps, in_sc, dout_sc,
+  wgrad16_kernel<BN, NP><<<(unsigned)(2 * clusters), kThreadsW16, C::SMEM, st>>>(P, maps, in_sc, dout_sc,
                                                                            dw, ws);
   EPB_LAUNCH_CHECK();
   if (P.splits > 1) {
@@ -268,10 +279,11 @@ int launch_w16(const PlanW16& P, const MapsW16& maps, const float* in_sc, const 
 
 extern "C" __attribute__((visibility("default"))) int epb_conv16_wgrad(
     const epb_conv_geom* g, const epb_half* in, const float* in_sc, const epb_half* dout,
-    const float* dout_sc, float* dw, float* ws, long long ws_floats, epb_stream_t stream) {
+    const float* dout_sc, float* dw, float* ws, long long ws_floats, int planes, epb_stream_t stream) {
   int rc = epb_conv_geom_check(g);
   if (rc) return rc;
   EPB_CHECK_ARG(in && in_sc && dout && dout_sc && dw);
+  EPB_CHECK_ARG(planes == 1 || planes == 2);
   EPB_CHECK_ARG(g->Cin % 64 == 0 && g->Cout % 64 == 0);
   EPB_CHECK_ARG((g->is == 1 || g->is == 2) && (g->os == 1 || g->os == 2));
   PlanW16 P;
@@ -314,7 +326,8 @@ extern "C" __attribute__((visibility("default"))) int epb_conv16_wgrad(
   memset(in_maps, 0, sizeof(in_maps));
   for (int v = 0; v < 4; ++v) {
     if (!need[v]) continue;
-    rc = epb_make_act_map(&in_maps[v], in, N, Hi, Wi, g->Cin, g->is, v >> 1, v & 1, P.tw, P.th, P.tn);
+    rc = epb_make_act_map(&in_maps[v], in, N, Hi, Wi, g->Cin, g->is, v >> 1, v & 1, P.tw, P.th, P.tn,
+                          planes);
     if (rc) return rc;
   }
   for (int v = 0; v < 4; ++v)
@@ -323,7 +336,7 @@ extern "C" __attribute__((visibility("default"))) int epb_conv16_wgrad(
         if (need[u]) { in_maps[v] = in_maps[u]; break; }
     }
   CUtensorMap d_map;
-  rc = epb_make_act_map(&d_map, dout, N, Ho, Wo, g->Cout, g->os, g->ph, g->pw, P.tw, P.th, P.tn);
+  rc = epb_make_act_map(&d_map, dout, N, Ho, Wo, g->Cout, g->os, g->ph, g->pw, P.tw, P.th, P.tn, planes);
   if (rc) return rc;
   int bn;
   if (!P.swap) {
@@ -354,6 +367,10 @@ extern "C" __attribute__((visibility("default"))) int epb_conv16_wgrad(
   P.tiles_per_split = (int)((P.ptiles + splits - 1) / splits);
   P.splits = (P.ptiles + P.tiles_per_split - 1) / P.tiles_per_split;
   cudaStream_t st = as_stream(stream);
-  if (bn == 128) return launch_w16<128>(P, maps, in_sc, dout_sc, dw, ws, st);
-  return launch_w16<256>(P, maps, in_sc, dout_sc, dw, ws, st);
+  if (planes == 1) {
+    if (bn == 128) return launch_w16<128, 1>(P, maps, in_sc, dout_sc, dw, ws, st);
+    return launch_w16<256, 1>(P, maps, in_sc, dout_sc, dw, ws, st);
+  }
+  if (bn == 128) return launch_w16<128, 2>(P, maps, in_sc, dout_sc, dw, ws, st);
+  return launch_w16<256, 2>(P, maps, in_sc, dout_sc, dw, ws, st);
 }

@@ -9,6 +9,10 @@ ValueError exactly like reference :167,184.
 Extra keys (superset, all default-off): TRAIN.ONLINE_TRIANGULATION,
 TRAIN.TRIANGULATION_METHOD, TRAIN.CUDA_GRAPH (default on), MODEL.PRECISION,
 DATASET.SYNTHETIC_LEN.
+
+MODEL.PRECISION (lib/models/pose3d_resnet.py; EPB_PRECISION overrides it): f16x3 (fp32-grade,
+three fp16 tensor passes over hi/lo operand planes), f16 (one fp16 pass over the hi planes:
+TF32-class operands, the fastest mode), tf32x3, tf32 (single pass), fp32.
 """
 import os
 

@@ -73,11 +73,12 @@ class _SoftArgmaxFn(torch.autograd.Function):
         if sink is not None and not sink.filled:
             # the gradient goes to the network's backward as split planes + bias gradient; autograd
             # carries a zero token (see _sinks.py)
-            sink.planes = torch.empty((2,) + tuple(st.shape), device=st.device, dtype=torch.float16)
+            sink.planes = torch.empty((sink.nplanes,) + tuple(st.shape), device=st.device, dtype=torch.float16)
             sink.sc = torch.empty(2, device=st.device, dtype=torch.float32)
             sink.dbias = torch.empty(J * D, device=st.device, dtype=torch.float32)
             ops.softargmax_bwd_split(st, N, J, D, H, W, coords, lse, dcoords.contiguous(), sink.planes,
-                                     sink.sc, sink.dbias)
+                                     sink.sc, sink.dbias,
+                                     **({} if sink.nplanes == 2 else {"planes": sink.nplanes}))
             sink.filled = True
             return sink.token.expand(preds.shape), None, None, None, None
         dst = torch.empty_like(st)

@@ -26,8 +26,12 @@ BN_MOMENTUM = 0.1
 logger = logging.getLogger(__name__)
 
 # f16x3: split-fp16 operands, three kind::f16 tensor passes (net16.Engine16); plans with
-# channel counts outside whole 64-element TMA boxes keep the 3xTF32 engine
-_PRECISIONS = {"fp32": 0, "tf32": 1, "tf32x3": 3, "f16x3": 4}
+# channel counts outside whole 64-element TMA boxes keep the 3xTF32 engine.
+# f16: the same engine on the hi planes alone, one kind::f16 pass (TF32-class operands); its
+# fall-back for such plans is the single-pass TF32 engine.
+_PRECISIONS = {"fp32": 0, "tf32": 1, "tf32x3": 3, "f16x3": 4, "f16": 5}
+_SPLIT_PLANES = {4: 2, 5: 1}           # Engine16 plane count of the split precisions
+_FALLBACK = {4: 3, 5: 1}               # net.Engine precision when net16 does not take the plan
 DEFAULT_PRECISION = "f16x3"
 
 
@@ -113,7 +117,7 @@ class _PoseNetFn(torch.autograd.Function):
             elif need_grad and module.training and module.fused_head_gradient \
                     and getattr(eng, "takes_logit_sink", lambda: False)():
                 # the criterion may hand the logit gradient over as split planes (_sinks.py)
-                ctx.sink = module._last_sink = _sinks.LogitGradSink(out)
+                ctx.sink = module._last_sink = _sinks.LogitGradSink(out, eng.planes)
             return out
         hm = torch.empty((N, fin.cout, Ho, Wo), device=x.device, dtype=torch.float32)
         eng.ops.nhwc_to_nchw(logits, hm, N, fin.cout, Ho, Wo, Cp)
@@ -138,8 +142,7 @@ class _PoseNetFn(torch.autograd.Function):
             else:
                 # the logits had other consumers too: their (fp32) gradients accumulated onto the
                 # zero token; add the sink's share back and take the fp32 route
-                share = (sink.planes[0].float() + sink.planes[1].float()) * sink.sc[1]
-                g0 = g0 + share.permute(0, 3, 1, 2)
+                g0 = g0 + sink.dense().permute(0, 3, 1, 2)
         nhwc = g0.permute(0, 2, 3, 1)
         if head is not None:
             dlogits = None
@@ -284,10 +287,10 @@ class PoseResNet(nn.Module):
     # ---- compute
     def _engine(self):
         if self._eng is None or self._eng_precision != self.precision:
-            if self.precision == 4 and _net16.supported(self._plan):
-                self._eng = _net16.Engine16(self._plan, ops=self._ops)
+            if self.precision in _SPLIT_PLANES and _net16.supported(self._plan):
+                self._eng = _net16.Engine16(self._plan, ops=self._ops, planes=_SPLIT_PLANES[self.precision])
             else:
-                self._eng = _net.Engine(self._plan, precision=3 if self.precision == 4 else self.precision,
+                self._eng = _net.Engine(self._plan, precision=_FALLBACK.get(self.precision, self.precision),
                                         ops=self._ops)
             self._eng_precision = self.precision
         return self._eng

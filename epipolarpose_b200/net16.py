@@ -15,6 +15,11 @@ epilogue output, accumulate target of the residual joins); gradients w.r.t. conv
 BatchNorm-backward reductions; the fp32 logit gradient that enters the network's backward is
 split once (amax + split).  Heads whose channel count is not a whole number of 64-channel blocks
 (test-sized) keep their backward on the 3xTF32 kernels of net.Engine.
+
+planes=1 is the single-pass "f16" mode: every split tensor is its hi plane alone (the TF32
+operand class: 10 explicit mantissa bits, power-of-two scale as above), the GEMMs issue one
+kind::f16 pass per k-step, no lo plane is ever written, and the fp32-operand layers run
+single-pass TF32 instead of 3xTF32.
 """
 import os
 
@@ -41,23 +46,30 @@ def supported(plan):
 
 class Engine16(_net.Engine):
 
-    def __init__(self, plan, ops=None):
-        super().__init__(plan, precision=3, ops=ops)   # 3xTF32 for the few fp32-operand layers
-        self.tc_precision = 3
+    def __init__(self, plan, ops=None, planes=2):
+        if planes not in (1, 2):
+            raise ValueError("planes must be 1 (f16) or 2 (f16x3), got %r" % (planes,))
+        # the few fp32-operand layers: 3xTF32 beside three f16 passes, TF32 beside one
+        prec = 3 if planes == 2 else 1
+        super().__init__(plan, precision=prec, ops=ops)
+        self.tc_precision = prec
+        self.planes = planes
+        # plane count for the split-family calls; the two-plane calls pass none (the default)
+        self._pk = {} if planes == 2 else {"planes": planes}
         # the fp32 packed weights are only read by the amax / split passes and the packed weight gradients
         # only written by plain stores: 1x1 layers use the parameter / gradient tensors themselves
         self.alias_1x1 = True
         self.stem_kpad = STEM_KPAD16
         self.stem_col = Conv("conv1", "conv", STEM_KPAD16, 64, 1, 1, 0)
 
-    # geometry tables are shared with the 3xTF32 kernels: their precision field must be 3
+    # geometry tables are shared with the fp32-operand kernels: their precision field is theirs
     def _geoms(self, conv, kind, N, H, W):
         f = conv.fprop_geoms if kind == "f" else conv.dgrad_geoms
         return f(self.ops, N, H, W, self.tc_precision)
 
     # ------------------------------------------------------------------ persistent state
     def _half(self, *shape):
-        return torch.empty((2,) + tuple(shape), device=self.dev, dtype=torch.float16)
+        return torch.empty((self.planes,) + tuple(shape), device=self.dev, dtype=torch.float16)
 
     def _consts(self):
         st = getattr(self, "_cst", None)
@@ -85,12 +97,12 @@ class Engine16(_net.Engine):
                     if t is None:
                         ent.append(None)
                         continue
-                    h = torch.empty(2 * t.numel(), device=self.dev, dtype=torch.float16)
+                    h = torch.empty(self.planes * t.numel(), device=self.dev, dtype=torch.float16)
                     sc = torch.ones(2, device=self.dev, dtype=torch.float32)
                     jobs.append((t, h, sc))
                     ent.append((h, sc))
                 out[name] = tuple(ent)
-            st = {"key": key, "w": out, "batch": ops.SplitBatch(jobs)}
+            st = {"key": key, "w": out, "batch": ops.SplitBatch(jobs, **self._pk)}
             self._w16 = st
         ops.split16_batch(st["batch"])
         return st["w"]
@@ -107,7 +119,7 @@ class Engine16(_net.Engine):
             if g is None:
                 continue
             g.in_relu, g.accumulate = 0, 0
-            ops.conv16_fprop(g, x, x_sc, w16[0], w16[1], out, bias, stats)
+            ops.conv16_fprop(g, x, x_sc, w16[0], w16[1], out, bias, stats, **self._pk)
         return out, Ho, Wo
 
     def _conv_dgrad16(self, conv, dz, dz_sc, N, H, W, wd16, accumulate_into=None):
@@ -124,7 +136,7 @@ class Engine16(_net.Engine):
                 continue
             g.in_relu = 0
             g.accumulate = 1 if accumulate_into is not None else 0
-            ops.conv16_fprop(g, dz, dz_sc, wd16[0], wd16[1], din, None, None)
+            ops.conv16_fprop(g, dz, dz_sc, wd16[0], wd16[1], din, None, None, **self._pk)
         return din
 
     def _conv_wgrad16(self, conv, x, x_sc, dz, dz_sc, N, H, W):
@@ -139,7 +151,7 @@ class Engine16(_net.Engine):
                 if g is None:
                     continue
                 g.in_relu, g.accumulate = 0, 0
-                ops.conv16_wgrad(g, x, x_sc, dz, dz_sc, dwp, ws)
+                ops.conv16_wgrad(g, x, x_sc, dz, dz_sc, dwp, ws, **self._pk)
 
         side = getattr(self, "_side", None)
         if side is None:
@@ -161,7 +173,8 @@ class Engine16(_net.Engine):
         dz_sc = torch.empty(2, device=self.dev, dtype=torch.float32)
         ops.bn_bwd_split(dy, z, None, st.scale, st.shift, st.mean, st.invstd,
                          params[st.name + ".weight"], relu, M, C, dz, dz_sc, dy_masked,
-                         grads[st.name + ".weight"], grads[st.name + ".bias"], mask_bits=mask_bits)
+                         grads[st.name + ".weight"], grads[st.name + ".bias"], mask_bits=mask_bits,
+                         **self._pk)
         return dz, dz_sc
 
     # ------------------------------------------------------------------ forward
@@ -217,7 +230,7 @@ class Engine16(_net.Engine):
             sc = new_sc()
             st = bn(name, C, M, sc)
             a = self._half(*shape)
-            ops.bn_act_split(z, st.scale, st.shift, None, None, None, None, None, 1, M, C, a, sc)
+            ops.bn_act_split(z, st.scale, st.shift, None, None, None, None, None, 1, M, C, a, sc, **self._pk)
             return st, a, sc
 
         # ---- stem (pose3d_resnet.py:186-189): patch matrix -> 1x1 GEMM -> BN+ReLU+maxpool
@@ -225,14 +238,14 @@ class Engine16(_net.Engine):
         H1, W1 = stem.out_hw(H, W)
         col = self._half(N, H1, W1, kpad)
         isc = cst["img_sc"]
-        ops.im2col_split(x_nchw, col, isc, N, 3, H, W, 7, 7, 2, 3, H1, W1, kpad)
+        ops.im2col_split(x_nchw, col, isc, N, 3, H, W, 7, 7, 2, 3, H1, W1, kpad, **self._pk)
         z0, _, _ = self._conv_fwd16(scol, col, isc, N, H1, W1, w16(stem), stats=stats_of("bn1", 64))
         cur_sc = new_sc()
         b0 = bn("bn1", 64, N * H1 * W1, cur_sc)
         H2, W2 = (H1 + 2 - 3) // 2 + 1, (W1 + 2 - 3) // 2 + 1
         cur = self._half(N, H2, W2, 64)
         argidx = torch.empty((N, H2, W2, 64), device=self.dev, dtype=torch.uint8)
-        ops.bn_relu_maxpool_split(z0, b0.scale, b0.shift, cur, cur_sc, argidx, N, H1, W1, 64)
+        ops.bn_relu_maxpool_split(z0, b0.scale, b0.shift, cur, cur_sc, argidx, N, H1, W1, 64, **self._pk)
         S["stem"] = (col, z0, argidx, H1, W1, H2, W2)
         h, w = H2, W2
 
@@ -268,11 +281,11 @@ class Engine16(_net.Engine):
                 rec["zd"] = zd
                 last = bn(lname, Cl, M, out_sc, (stats_of(dname, dC), dst.scale, dst.shift))
                 ops.bn_act_split(zl, last.scale, last.shift, zd, dst.scale, dst.shift, None, None,
-                                 1, M, Cl, out, out_sc, obits)
+                                 1, M, Cl, out, out_sc, obits, **self._pk)
             else:
                 last = bn(lname, Cl, M, out_sc, res_sc=cur_sc)
                 ops.bn_act_split(zl, last.scale, last.shift, None, None, None, cur, cur_sc, 1, M, Cl,
-                                 out, out_sc, obits)
+                                 out, out_sc, obits, **self._pk)
             rec["out"] = (out, out_sc)
             rec["mask"] = obits
             S["blocks"].append(rec)
@@ -300,7 +313,7 @@ class Engine16(_net.Engine):
             fbias = fb
         logits, ho, wo = self._conv_fwd16(fin, src, src_sc, N, h, w, w16(fin), bias=fbias)
         # the final layer's backward: split operands when the head has whole 64-channel blocks,
-        # else the 3xTF32 kernels from (z, BatchNorm affine)
+        # else the fp32-operand kernels from (z, BatchNorm affine)
         S["final"] = (zlast, (stlast.scale, stlast.shift), h, w)
         S["final16"] = (src, src_sc)
         depth = None
@@ -308,7 +321,7 @@ class Engine16(_net.Engine):
             tr, tr_sc, th, tw = S["trunk"]
             assert th == plan.pool_k and tw == plan.pool_k, "AvgPool(k) -> 1x1 expected"
             pooled = torch.empty((N, 1, 1, 2048), device=self.dev, dtype=torch.float32)
-            ops.avgpool_split(tr, tr_sc, pooled, N, th * tw, 2048)
+            ops.avgpool_split(tr, tr_sc, pooled, N, th * tw, 2048, **self._pk)
             depth, _, _ = self._conv_fwd(plan.fc, pooled, N, 1, 1, S["packed"][plan.fc.name][0],
                                          bias=params["depth_fc.bias"])
             S["fc"] = pooled
@@ -360,12 +373,12 @@ class Engine16(_net.Engine):
                 # gradient on the split kernels like every other layer (deterministic)
                 dl16 = self._half(N, Ho, Wo, fin.cout_p)
                 dl_sc = torch.empty(2, device=self.dev, dtype=torch.float32)
-                ops.split16(dlogits.reshape(-1), dl16.reshape(-1), dl_sc, self._consts()["amax1"])
+                ops.split16(dlogits.reshape(-1), dl16.reshape(-1), dl_sc, self._consts()["amax1"], **self._pk)
             fsrc, fsrc_sc = S["final16"]
             self._conv_wgrad16(fin, fsrc, fsrc_sc, dl16, dl_sc, N, h, w)
             dcur = self._conv_dgrad16(fin, dl16, dl_sc, N, h, w, wd16(fin))
         else:
-            # few output channels (test-sized heads): the 3xTF32 kernels take the fp32 gradient
+            # few output channels (test-sized heads): the fp32-operand kernels take the fp32 gradient
             self._conv_wgrad(fin, src, dlogits, N, h, w, grads[fin.name + ".weight"], affine=aff)
             dcur = self._conv_dgrad(fin, dlogits, N, h, w, S["packed"][fin.name][1])
         # ---- deconv head, reversed

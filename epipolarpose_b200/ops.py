@@ -189,7 +189,8 @@ def colsum(x, M, C, out):
 
 # ------------------------------------------------------------------ split-fp16 ("f16x3") family
 # A split tensor is a torch.float16 tensor [2, ...] (hi plane, lo plane) plus a device
-# float32[2] = (s, 1/s).
+# float32[2] = (s, 1/s).  `planes=1` selects the single-pass layout [1, ...] (hi plane only,
+# include/epb.h): producers write the hi plane alone, readers and GEMMs read it alone.
 
 _H = torch.float16
 
@@ -206,33 +207,35 @@ def bn_finalize_scale(stats, M, C, gamma, beta, eps, momentum, running_mean, run
           _p(stats2, torch.float64), _p(scale2), _p(shift2), _p(res_sc), _p(sc), _stream())
 
 
-def bn_act_split(x, scale, shift, r, rscale, rshift, r_split, r_sc, relu, M, C, y, y_sc, mask_bits=None):
+def bn_act_split(x, scale, shift, r, rscale, rshift, r_split, r_sc, relu, M, C, y, y_sc, mask_bits=None,
+                 planes=2):
     _call("epb_bn_act_split", _p(x), _p(scale), _p(shift), _p(r), _p(rscale), _p(rshift),
           _p(r_split, _H), _p(r_sc), int(relu), M, C, _p(y, _H), _p(y_sc), _p(mask_bits, torch.uint8),
-          _stream())
+          planes, _stream())
 
 
-def bn_relu_maxpool_split(x, scale, shift, y, y_sc, argidx, N, H, W, C):
+def bn_relu_maxpool_split(x, scale, shift, y, y_sc, argidx, N, H, W, C, planes=2):
     _call("epb_bn_relu_maxpool_split", _p(x), _p(scale), _p(shift), _p(y, _H), _p(y_sc),
-          _p(argidx, torch.uint8), N, H, W, C, _stream())
+          _p(argidx, torch.uint8), N, H, W, C, planes, _stream())
 
 
-def im2col_split(img, col, col_sc, N, C, Hi, Wi, kh, kw, stride, pad, Ho, Wo, Kpad):
+def im2col_split(img, col, col_sc, N, C, Hi, Wi, kh, kw, stride, pad, Ho, Wo, Kpad, planes=2):
     _call("epb_im2col_split", _p(img), _p(col, _H), _p(col_sc), N, C, Hi, Wi, kh, kw, stride, pad,
-          Ho, Wo, Kpad, _stream())
+          Ho, Wo, Kpad, planes, _stream())
 
 
 class SplitBatch:
     """A fixed list of fp32 -> split conversions (epb_split_job) with its device table.
-    jobs: (src fp32 [n], dst fp16 [2][n], sc fp32 [2]); the tensors must stay where they are."""
+    jobs: (src fp32 [n], dst fp16 [planes][n], sc fp32 [2]); the tensors must stay where they are."""
 
-    def __init__(self, jobs):
+    def __init__(self, jobs, planes=2):
         import struct
         self.jobs = list(jobs)
+        self.planes = planes
         blob, first = b"", 0
         for (src, dst, sc) in self.jobs:
             n = src.numel()
-            assert dst.numel() == 2 * n and dst.dtype == _H and sc.numel() == 2
+            assert dst.numel() == planes * n and dst.dtype == _H and sc.numel() == 2
             blob += struct.pack("<QQQqq", src.data_ptr(), dst.data_ptr(), sc.data_ptr(), n, first)
             first += (n + 2047) // 2048
         self.total_blocks = first
@@ -241,23 +244,24 @@ class SplitBatch:
         self.amax = torch.zeros(len(self.jobs), dtype=torch.int32, device=dev)
 
 
-def split16(src, dst, sc, amax_ws):
-    _call("epb_split16", _p(src), src.numel(), _p(dst, _H), _p(sc), _p(amax_ws, torch.int32), _stream())
+def split16(src, dst, sc, amax_ws, planes=2):
+    _call("epb_split16", _p(src), src.numel(), _p(dst, _H), _p(sc), _p(amax_ws, torch.int32), planes,
+          _stream())
 
 
 def split16_batch(batch):
     _call("epb_split16_batch", _p(batch.table, torch.uint8), len(batch.jobs), batch.total_blocks,
-          _p(batch.amax, torch.int32), _stream())
+          _p(batch.amax, torch.int32), batch.planes, _stream())
 
 
-def conv16_fprop(g, x, x_sc, w, w_sc, out, bias=None, stats=None):
+def conv16_fprop(g, x, x_sc, w, w_sc, out, bias=None, stats=None, planes=2):
     _call("epb_conv16_fprop", ctypes.byref(g), _p(x, _H), _p(x_sc), _p(w, _H), _p(w_sc), _p(bias),
-          _p(out), _p(stats, torch.float64), _stream())
+          _p(out), _p(stats, torch.float64), planes, _stream())
 
 
-def conv16_wgrad(g, x, x_sc, dout, dout_sc, dw, ws):
+def conv16_wgrad(g, x, x_sc, dout, dout_sc, dw, ws, planes=2):
     _call("epb_conv16_wgrad", ctypes.byref(g), _p(x, _H), _p(x_sc), _p(dout, _H), _p(dout_sc),
-          _p(dw), _p(ws), ws.numel() if ws is not None else 0, _stream())
+          _p(dw), _p(ws), ws.numel() if ws is not None else 0, planes, _stream())
 
 
 def bn_bwd_reduce_mx(dy, x, mask_hi, scale, shift, mean, invstd, relu, M, C, sums, maxes):
@@ -266,22 +270,22 @@ def bn_bwd_reduce_mx(dy, x, mask_hi, scale, shift, mean, invstd, relu, M, C, sum
 
 
 def bn_bwd_apply_split(dy, x, mask_hi, scale, shift, mean, invstd, gamma, relu, sums, maxes, M, C,
-                       dz, dz_sc, dy_masked, dgamma, dbeta):
+                       dz, dz_sc, dy_masked, dgamma, dbeta, planes=2):
     _call("epb_bn_bwd_apply_split", _p(dy), _p(x), _p(mask_hi, _H), _p(scale), _p(shift), _p(mean),
           _p(invstd), _p(gamma), int(relu), _p(sums, torch.float64), _p(maxes), M, C, _p(dz, _H),
-          _p(dz_sc), _p(dy_masked), _p(dgamma), _p(dbeta), _stream())
+          _p(dz_sc), _p(dy_masked), _p(dgamma), _p(dbeta), planes, _stream())
 
 
 def bn_bwd_split(dy, x, mask_hi, scale, shift, mean, invstd, gamma, relu, M, C, dz, dz_sc, dy_masked,
-                 dgamma, dbeta, mask_bits=None):
+                 dgamma, dbeta, mask_bits=None, planes=2):
     _call("epb_bn_bwd_split", _p(dy), _p(x), _p(mask_hi, _H), _p(mask_bits, torch.uint8), _p(scale),
           _p(shift), _p(mean),
           _p(invstd), _p(gamma), int(relu), M, C, _p(dz, _H), _p(dz_sc), _p(dy_masked), _p(dgamma),
-          _p(dbeta), _stream())
+          _p(dbeta), planes, _stream())
 
 
-def avgpool_split(x, x_sc, y, N, HW, C):
-    _call("epb_avgpool_split", _p(x, _H), _p(x_sc), _p(y), N, HW, C, _stream())
+def avgpool_split(x, x_sc, y, N, HW, C, planes=2):
+    _call("epb_avgpool_split", _p(x, _H), _p(x_sc), _p(y), N, HW, C, planes, _stream())
 
 
 # ------------------------------------------------------------------ decode / loss
@@ -311,9 +315,9 @@ def argmax2d(hm, NJ, H, W, idx, maxval, preds):
     _call("epb_argmax2d", _p(hm), NJ, H, W, _p(idx, torch.int32), _p(maxval), _p(preds), _stream())
 
 
-def softargmax_bwd_split(logits, N, J, D, H, W, coords, lse, dcoords, dlogits16, sc, dbias):
+def softargmax_bwd_split(logits, N, J, D, H, W, coords, lse, dcoords, dlogits16, sc, dbias, planes=2):
     _call("epb_softargmax_bwd_split", _p(logits), N, J, D, H, W, _p(coords), _p(lse), _p(dcoords),
-          _p(dlogits16, _H), _p(sc), _p(dbias), _stream())
+          _p(dlogits16, _H), _p(sc), _p(dbias), planes, _stream())
 
 
 def final_preds(hm, N, J, H, W, center, scale, post_process, preds, maxvals):

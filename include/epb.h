@@ -200,6 +200,13 @@ int epb_colsum(const float* x, int64_t M, int C, float* out,
  * s a power of two), planes[0] = hi, planes[1] = lo, each [rows][C] fp16 (raw bits,
  * epb_half), C % 8 == 0; `sc` is a DEVICE float[2] = {s, 1/s}.  Three tensor passes
  * (lo*hi + hi*lo + hi*hi, fp32 accumulation) reproduce the fp32 product to ~2^-22.
+ *
+ * Single-pass layout ("f16"): `int planes` = 1 on the calls below selects [1][rows][C], the
+ * hi plane alone (x*s ~= hi: 10 explicit mantissa bits, the TF32 operand class).  Producers
+ * then write neither the lo plane nor its address range (the buffer may end after the hi
+ * plane), readers read hi only, and the GEMMs issue one kind::f16 pass (hi*hi) per k-step.
+ * Scales and bounds are those of the two-plane form.  planes = 2 is the layout above; the
+ * plane count is a launch argument (the GEMMs build their TMA tensor maps from it).
  * ---------------------------------------------------------------------- */
 typedef uint16_t epb_half;
 
@@ -228,22 +235,22 @@ int epb_bn_act_split(const float* x, const float* scale, const float* shift,
                      const float* r, const float* rscale, const float* rshift,
                      const epb_half* r_split, const float* r_sc, int relu,
                      int64_t M, int C, epb_half* y, const float* y_sc,
-                     uint8_t* mask_bits, epb_stream_t stream);
+                     uint8_t* mask_bits, int planes, epb_stream_t stream);
 /* mask_bits (optional, [M*C/8] bytes): bit k of byte i = (pre-ReLU value of element 8*i+k > 0),
  * the ReLU mask the BatchNorm backward of the block reads (epb_bn_bwd_split). */
 /* stem: maxpool3x3s2p1(relu(x*scale+shift)) -> split tensor + argmax slot (0..8) */
 int epb_bn_relu_maxpool_split(const float* x, const float* scale, const float* shift,
                               epb_half* y, const float* y_sc, uint8_t* argidx, int N,
-                              int H, int W, int C, epb_stream_t stream);
+                              int H, int W, int C, int planes, epb_stream_t stream);
 /* patch matrix of the 7x7 stem straight from the NCHW image (pose3d_resnet.py:99,185):
  * col[m][(r*kw+s)*C + c] = img[n][c][oh*stride-pad+r][ow*stride-pad+s], zero padded to
- * Kpad (% 64 == 0) columns, as a split tensor [2][N*Ho*Wo][Kpad]. */
+ * Kpad (% 64 == 0) columns, as a split tensor [planes][N*Ho*Wo][Kpad]. */
 int epb_im2col_split(const float* img_nchw, epb_half* col, const float* col_sc, int N,
                      int C, int Hi, int Wi, int kh, int kw, int stride, int pad, int Ho,
-                     int Wo, int Kpad, epb_stream_t stream);
+                     int Wo, int Kpad, int planes, epb_stream_t stream);
 /* fp32 tensors -> split tensors with a per-tensor power-of-two scale chosen from the
  * tensor's max |x| (largest scaled magnitude in [2^13, 2^14)); job j: src[n] ->
- * dst[2][n], sc[2] written.  Blocks of 2048 elements, jobs ordered by first_block.
+ * dst[planes][n], sc[2] written.  Blocks of 2048 elements, jobs ordered by first_block.
  * amax_ws: njobs uint32 of DEVICE scratch (zeroed by the call). */
 typedef struct epb_split_job {
   const float* src;
@@ -253,33 +260,34 @@ typedef struct epb_split_job {
   long long first_block;
 } epb_split_job;
 int epb_split16_batch(const epb_split_job* jobs, int njobs, long long total_blocks,
-                      uint32_t* amax_ws, epb_stream_t stream);
+                      uint32_t* amax_ws, int planes, epb_stream_t stream);
 
 /* one tensor (n % 4 == 0), pointers as arguments: for tensors whose address is only known at
  * call time (the logit gradient autograd hands to the network's backward).  amax_ws: one
  * uint32 of DEVICE scratch. */
 int epb_split16(const float* src, long long n, epb_half* dst, float* sc, uint32_t* amax_ws,
-                epb_stream_t stream);
+                int planes, epb_stream_t stream);
 
-/* epb_conv_fprop on split operands: in [2][N,Hi,Wi,Cin], w [2][Cout][Tw*Cin] (the packed
+/* epb_conv_fprop on split operands: in [planes][N,Hi,Wi,Cin], w [planes][Cout][Tw*Cin] (the packed
  * operand of epb_pack_weight, split).  Cin % 64 == 0, Cout % 4 == 0.  CTA pairs
  * (tcgen05 cta_group::2, M = 256), A and B tiles by TMA (5-D / 3-D tensor maps; the
  * zero padding of the convolution is the TMA out-of-bounds fill), fp32 accumulators
  * in TMEM; out = acc / (s_in * s_w) (+ bias), optional accumulate / statistics as
- * epb_conv_fprop.  g->precision, g->in_relu are ignored (operands are post-activation). */
+ * epb_conv_fprop.  g->precision, g->in_relu are ignored (operands are post-activation).
+ * planes 2: three kind::f16 passes; planes 1: one pass over the hi planes. */
 int epb_conv16_fprop(const epb_conv_geom* g, const epb_half* in, const float* in_sc,
                      const epb_half* w, const float* w_sc, const float* bias,
-                     float* out, double* stats, epb_stream_t stream);
-/* epb_conv_wgrad on split operands (in as above, dout [2][N,Ho,Wo,Cout]); both operands
+                     float* out, double* stats, int planes, epb_stream_t stream);
+/* epb_conv_wgrad on split operands (in as above, dout [planes][N,Ho,Wo,Cout]); both operands
  * MN-major by TMA, reduction over pixel tiles split across clusters and summed in a FIXED
  * order from `ws` (deterministic): dw[co][wt[t]][ci] += sum.  ws: >= ws_floats floats of
  * scratch (the call uses as many split partials as fit). */
 int epb_conv16_wgrad(const epb_conv_geom* g, const epb_half* in, const float* in_sc,
                      const epb_half* dout, const float* dout_sc, float* dw, float* ws,
-                     long long ws_floats, epb_stream_t stream);
+                     long long ws_floats, int planes, epb_stream_t stream);
 
 /* BatchNorm(+ReLU) backward for the split path.  mask = (mask_hi > 0) when mask_hi != NULL
- * (hi plane of the block output), else (x*scale+shift > 0) if relu, else 1.
+ * (hi plane of the block output, of either layout: only the hi plane is read), else (x*scale+shift > 0) if relu, else 1.
  * reduce: sums as epb_bn_bwd_reduce; maxes[0..C) = max |g|, maxes[C..2C) = max |xhat|
  *         (float, caller zeroes; used to bound |dz| for the scale of the split output).
  *         Two launches: per-CTA partials, then a fixed-order combine (deterministic).
@@ -296,7 +304,7 @@ int epb_bn_bwd_apply_split(const float* dy, const float* x, const epb_half* mask
                            const float* invstd, const float* gamma, int relu,
                            const double* sums, const float* maxes, int64_t M, int C,
                            epb_half* dz, float* dz_sc, float* dy_masked, float* dgamma,
-                           float* dbeta, epb_stream_t stream);
+                           float* dbeta, int planes, epb_stream_t stream);
 /* Both passes in one call (what the engine uses): per-CTA partial reductions, a fixed-order
  * combine (no atomics: dgamma / dbeta / the scale of dz are run-to-run identical), apply.
  * Outputs as epb_bn_bwd_apply_split; the sums / maxes live in internal scratch of the stream.
@@ -305,10 +313,10 @@ int epb_bn_bwd_apply_split(const float* dy, const float* x, const epb_half* mask
 int epb_bn_bwd_split(const float* dy, const float* x, const epb_half* mask_hi,
                      const uint8_t* mask_bits, const float* scale, const float* shift, const float* mean, const float* invstd,
                      const float* gamma, int relu, int64_t M, int C, epb_half* dz, float* dz_sc,
-                     float* dy_masked, float* dgamma, float* dbeta, epb_stream_t stream);
+                     float* dy_masked, float* dgamma, float* dbeta, int planes, epb_stream_t stream);
 /* VOLUME=False head on a split tensor: y[n][c] = mean over HW of x (fp32 out) */
 int epb_avgpool_split(const epb_half* x, const float* x_sc, float* y, int N, int HW, int C,
-                      epb_stream_t stream);
+                      int planes, epb_stream_t stream);
 
 /* ------------------------------------------------------------------------
  * Soft-argmax (ATen softmax + 9 reductions: lib/core/integral_loss.py:49-86)
@@ -327,14 +335,15 @@ int epb_softargmax_bwd(const float* logits, int layout, int N, int J, int D,
                        const float* dcoords, float* dlogits,
                        epb_stream_t stream);
 /* The same gradient written straight as the split operand of the final layer's backward
- * (channels_last logits only, D % 4 == 0, J*D/4 <= 1024): dlogits16 = planes [2][N][H][W][J*D],
+ * (channels_last logits only, D % 4 == 0, J*D/4 <= 1024): dlogits16 = planes [planes][N][H][W][J*D],
  * sc = {s, 1/s} with s from the hard bound max_nj p_max * (|gx|+|gy|+|gz|), and (optional)
  * dbias[J*D] = column sums of the gradient = the final layer's bias gradient, added in a fixed
  * order.  Replaces epb_softargmax_bwd + epb_split16 + epb_colsum of the fp32 form (the logit
  * gradient never exists in fp32: 1 read + 1 write of the volume instead of 4 + 2). */
 int epb_softargmax_bwd_split(const float* logits, int N, int J, int D, int H, int W,
                              const float* coords, const float* lse_ws, const float* dcoords,
-                             epb_half* dlogits16, float* sc, float* dbias, epb_stream_t stream);
+                             epb_half* dlogits16, float* sc, float* dbias, int planes,
+                             epb_stream_t stream);
 
 /* Fused joint-location loss (integral_loss.py:7-47): kind 0 = weighted MSE,
  * 1 = weighted L1, 2 = weighted SmoothL1(beta=1).  loss = sum(w*l(x-t))/div,
